@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W              # our arm (default)
     python bench.py --impl reference --gpus 1 --steps K --warmup W
     torchrun ... bench.py --gpus N ...                          # one rank per GPU
+    python bench.py ... --dump-outputs DIR     # + the last timed step's outputs as DIR/*.npy
 
 A "step" is one sync step of one batch: every env of the pool advances once.  Workload at
 N=1: BASELINE.json configs[1], CartPole-v1 with num_envs=65536 on one B200.  N>1 is weak
@@ -48,6 +49,7 @@ TASKS = {
 METRIC = "env steps/sec (whole box)"
 L2_BYTES = 126 * 1024 * 1024
 MAX_CHAIN = 4096          # steps per captured chain (2-4 kernel nodes each)
+DUMP_BYTES = 60 << 20     # --dump-outputs: .npy data under 64 MB, headers included
 # fp64 operations per HalfCheetah env step (5 mj_step), from the instruction counts of one
 # ncu capture of hc_thread_kernel (profiles/README.md): DFMA = 2, DADD / DMUL = 1
 HC_FLOP_PER_ENV_STEP = None
@@ -414,6 +416,25 @@ def run_config_line(torch, dist, task, n_total, world, rank, local, dev, steps, 
     return line
 
 
+def dump_outputs(pool, path):
+    """The output columns of `pool`'s last step, as a caller of the device path receives them,
+    to path/<key>.npy: float columns as they are, integer columns as float64, flags as
+    float32.  Above DUMP_BYTES only a fixed, seeded sample of env rows is written (the same
+    rows in every run; the info:env_id column says which)."""
+    cols = {k: v.cpu().numpy() for k, v in pool.outputs_torch().items()}
+    cols = {k: v if v.dtype.kind == "f" else v.astype(np.float64 if v.dtype.kind in "iu"
+                                                       else np.float32)
+            for k, v in cols.items()}
+    row = sum(v[0].nbytes for v in cols.values())
+    if row * pool.n > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(pool.n, DUMP_BYTES // row,
+                                                       replace=False))
+        cols = {k: v[keep] for k, v in cols.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, v in cols.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -453,13 +474,20 @@ def run_ours(args):
     pool.step_many_device(actions, 0, W, use_graph=False)   # W warm-up steps, direct launches
     pool.sync()
     if not args.profile:
-        # ~1 s of the same launches before the timed region: clocks are sampled under load
+        # ~1 s of the same launches before the timed region: clocks are sampled under load.
+        # The env state is put back afterwards, so that what the timed steps compute does not
+        # depend on how many steps fit into that second.
+        snapshot = pool.state_export()
         t_w = time.time()
         while time.time() - t_w < 1.0:
             pool.step_many_device(actions, 0, min(1024, actions.shape[0]), use_graph=use_graph)
             pool.sync()
+        pool.state_import(snapshot)
+        del snapshot
     ms_total = timer.run(K, lead)
     launches = timer.launches
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pool, args.dump_outputs)
     t_load1 = time.time()
     clocks = sampler.stop(t_load0, t_load1) if rank == 0 and not args.profile else None
     ms_per_step = ms_total / K
@@ -771,8 +799,10 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20000)
-    ap.add_argument("--warmup", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 20000; 100 with --impl reference)")
+    ap.add_argument("--warmup", type=int, default=None,
+                    help="untimed warm-up steps (default: 2000; 3 with --impl reference)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--task", default="CartPole-v1", choices=sorted(TASKS))
     ap.add_argument("--num-envs", type=int, default=65536, help="envs per GPU")
@@ -789,10 +819,19 @@ def main():
                     help="kernel loop only (for ncu): no clocks sampler, e2e or cpu legs")
     ap.add_argument("--profile-rollout", action="store_true",
                     help="with --profile: also run the fused rollout leg (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<key>.npy")
     args = ap.parse_args()
-    if args.impl == "reference":
-        if args.steps == 20000 and args.warmup == 2000:
-            args.steps, args.warmup = 100, 3
+    ref = args.impl == "reference"
+    if args.steps is None:
+        args.steps = 100 if ref else 20000
+    if args.warmup is None:
+        args.warmup = 3 if ref else 2000
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if ref and args.dump_outputs:
+        ap.error("--dump-outputs records our arm's outputs: not with --impl reference")
+    if ref:
         run_reference(args)
     else:
         run_ours(args)

@@ -1,5 +1,6 @@
 """Shared helpers for the parity tests (test infrastructure; may import oracle/)."""
 import glob
+import hashlib
 import json
 import os
 
@@ -31,6 +32,37 @@ def load_golden(name):
     meta = json.loads(str(z["meta"]))
     data = {k: z[k] for k in z.files if k != "meta"}
     return meta, data
+
+
+def space_desc(sp):
+    """JSON description of a gymnasium space or dm_env spec."""
+    d = {"type": type(sp).__name__, "shape": list(sp.shape or ()), "dtype": str(sp.dtype)}
+    for k in ("low", "high", "minimum", "maximum"):
+        if hasattr(sp, k):
+            d[k] = [float(x) for x in np.ravel(getattr(sp, k))]
+    for k in ("n", "start", "num_values"):
+        if hasattr(sp, k) and isinstance(getattr(sp, k), int):
+            d[k] = getattr(sp, k)
+    return d
+
+
+def jsonable(v):
+    """A config value as JSON would give it back (tuples and arrays as lists)."""
+    if isinstance(v, dict):
+        return {k: jsonable(x) for k, x in v.items()}
+    if isinstance(v, (list, tuple, np.ndarray)):
+        return [jsonable(x) for x in v]
+    return v.item() if isinstance(v, np.generic) else v
+
+
+def batch_digest(batch):
+    """64-bit digest of a batch: name, dtype, shape and bytes of every key, in name order."""
+    h = hashlib.blake2b(digest_size=8)
+    for k in sorted(batch):
+        a = np.ascontiguousarray(batch[k])
+        h.update(f"{k}|{a.dtype.str}|{a.shape}|".encode())
+        h.update(a.tobytes())
+    return int.from_bytes(h.digest(), "little")
 
 
 def random_actions(task, rng, shape_prefix, act_dtype=None):

@@ -1,22 +1,25 @@
-"""Run the REFERENCE's own Python layer (imported unmodified from /root/reference) on top of
-this repo's pybind11 extension modules and print a JSON report.  Executed in a subprocess by
-tests/test_reference_python_layer.py so that the stand-in optree / dm_env / gymnasium packages
-(tests/refstubs) never leak into the main test process.
+"""Record what the REFERENCE's own Python layer (envpool/python/*.py, registration.py and the
+family packages, imported unmodified from a reference checkout) makes of this repo's pybind11
+extension modules, as tests/golden/reference_python_layer.json -- the record that
+tests/test_reference_python_layer.py compares this repo's own layer against:
 
-What it shows: the drop-in boundary of SURVEY.md 8(b) holds from the reference's side -- its
-`py_env()` metaclasses, `EnvSpec` mixin, registry and `make_spec()` consume
+    python tests/ref_layer_check.py <reference checkout>
+
+optree / dm_env / gymnasium need not be installed: tests/refstubs holds stand-ins for the few
+names that layer uses.  What the layer consumes is the drop-in boundary of SURVEY.md 8(b): its
+`py_env()` metaclasses, `EnvSpec` mixin, registry and `make_spec()` read
 `_config_keys / _default_config_values / _state_keys / _action_keys / _state_spec /
 _action_spec` and the tuple constructor of OUR `_XxxEnvSpec` / `_XxxEnvPool` classes exactly
-as they consume the Bazel-built ones (INTEGRATION.md section 1)."""
+as they read the Bazel-built ones (INTEGRATION.md section 1)."""
 import importlib
 import json
 import os
 import sys
 
-sys.dont_write_bytecode = True  # /root/reference is read-only and must stay untouched
+sys.dont_write_bytecode = True  # the reference checkout is left untouched
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get("ENVPOOL_REFERENCE_ROOT", "/root/reference")
+GOLDEN = os.path.join(HERE, "golden", "reference_python_layer.json")
 
 FAMILIES = {
     # reference package            compiled module it imports            ours
@@ -26,30 +29,19 @@ FAMILIES = {
 }
 
 
-def space_desc(sp):
-    d = {"type": type(sp).__name__, "shape": list(sp.shape or ()), "dtype": str(sp.dtype)}
-    for k in ("low", "high", "minimum", "maximum"):
-        if hasattr(sp, k):
-            d[k] = [float(x) for x in __import__("numpy").ravel(getattr(sp, k))]
-    for k in ("n", "start", "num_values"):
-        if hasattr(sp, k) and isinstance(getattr(sp, k), int):
-            d[k] = getattr(sp, k)
-    return d
-
-
-def main():
+def main(ref):
     import numpy as np
+
+    from helpers import jsonable, space_desc
 
     sys.path.insert(0, ROOT)
     import envpool_b200  # noqa: F401  (ours, real spaces stand-ins of its own)
 
-    ours_specs = {}
     envpool_b200._ensure_registered()
     from envpool_b200.registration import registry as our_registry
 
-    report = {"tasks": {}, "errors": []}
     sys.path.insert(0, os.path.join(HERE, "refstubs"))
-    sys.path.insert(0, REF)
+    sys.path.insert(0, ref)
     for pkg, (mod, ours) in FAMILIES.items():
         sys.modules[f"{pkg}.{mod}"] = importlib.import_module(ours)
     # envpool/entry.py imports EVERY family's registration, and each family package imports
@@ -58,7 +50,7 @@ def main():
     import types
 
     sys.modules["envpool.entry"] = types.ModuleType("envpool.entry")
-    import envpool  # the reference package, from /root/reference
+    import envpool  # the reference package, from the checkout
     import envpool.classic_control.registration  # noqa: F401
     import envpool.toy_text.registration  # noqa: F401
 
@@ -70,7 +62,7 @@ def main():
 
     ours_mj = importlib.import_module("envpool_b200.mujoco.mujoco_gym_envpool")
     pkg = types.ModuleType("envpool.mujoco.gym")
-    pkg.__path__ = [os.path.join(REF, "envpool", "mujoco", "gym")]
+    pkg.__path__ = [os.path.join(ref, "envpool", "mujoco", "gym")]
     (pkg.GymHalfCheetahEnvSpec, pkg.GymHalfCheetahDMEnvPool,
      pkg.GymHalfCheetahGymnasiumEnvPool) = ref_py_env(ours_mj._GymHalfCheetahEnvSpec,
                                                       ours_mj._GymHalfCheetahEnvPool)
@@ -79,76 +71,44 @@ def main():
     sys.modules["envpool.mujoco.gym"] = pkg
     import envpool.mujoco.gym.registration  # noqa: F401
 
-    report["reference_file"] = envpool.__file__
-    ref_all = set(envpool.list_all_envs())
-    for task, (import_path, spec_cls, _) in sorted(our_registry.specs.items()):
+    assert os.path.abspath(envpool.__file__).startswith(os.path.abspath(ref))
+    report = {"reference": "sail-sg/envpool@9cbcd26",
+              "registry": sorted(envpool.list_all_envs()), "tasks": {}}
+    for task, (import_path, _, _) in sorted(our_registry.specs.items()):
         if not import_path.endswith(("classic_control", "toy_text", "mujoco.gym")):
             continue
-        entry = {"in_reference_registry": task in ref_all}
-        try:
-            rs = envpool.make_spec(task, num_envs=3, seed=11)
-            os_ = envpool_b200.make_spec(task, num_envs=3, seed=11)
-            rc, oc = rs.config._asdict(), os_.config._asdict()
-            # base_path is the install directory of whichever package registered the task
-            entry["base_path"] = [rc.pop("base_path", None), oc.pop("base_path", None)]
-            entry["config_equal"] = rc == oc
-            if rc != oc:
-                entry["config_diff"] = {k: (repr(rc.get(k)), repr(oc.get(k)))
-                                        for k in set(rc) | set(oc) if rc.get(k) != oc.get(k)}
-            entry["state_keys_equal"] = list(rs._state_keys) == list(os_._state_keys)
-            entry["action_keys_equal"] = list(rs._action_keys) == list(os_._action_keys)
-            ro, oo = rs.observation_space, os_.observation_space
-            entry["obs_space"] = space_desc(ro)
-            entry["obs_space_equal"] = (
-                list(ro.shape or ()) == list(oo.shape or ())
-                and all(np.array_equal(getattr(ro, k), getattr(oo, k))
-                        for k in ("low", "high") if hasattr(ro, k))
-                and getattr(ro, "n", None) == getattr(oo, "n", None))
-            ra, oa = rs.action_space, os_.action_space
-            entry["act_space"] = space_desc(ra)
-            entry["act_space_equal"] = (
-                list(ra.shape or ()) == list(oa.shape or ())
-                and all(np.array_equal(getattr(ra, k), getattr(oa, k))
-                        for k in ("low", "high") if hasattr(ra, k))
-                and getattr(ra, "n", None) == getattr(oa, "n", None))
-            dm_obs = rs.observation_spec()
-            entry["dm_obs_fields"] = list(dm_obs._fields)
-            entry["dm_action"] = space_desc(rs.action_spec())
-            entry["reward_threshold"] = rs.reward_threshold
-        except Exception as exc:  # noqa: BLE001
-            entry["error"] = f"{type(exc).__name__}: {exc}"
-            report["errors"].append(task)
-        report["tasks"][task] = entry
+        rs = envpool.make_spec(task, num_envs=3, seed=11)
+        rc = rs.config._asdict()
+        rc.pop("base_path", None)   # the install directory of the registering package
+        report["tasks"][task] = {
+            "config": jsonable(rc), "state_keys": list(rs._state_keys),
+            "action_keys": list(rs._action_keys),
+            "obs_space": space_desc(rs.observation_space),
+            "act_space": space_desc(rs.action_space),
+            "dm_obs_fields": list(rs.observation_spec()._fields),
+            "dm_action": space_desc(rs.action_spec()),
+            "reward_threshold": rs.reward_threshold}
 
-    # the reference's adapter classes built over OUR pool classes, and its dm fold
+    # the reference's dm fold over a batch in OUR column order
     import envpool.classic_control as rcc
 
-    cls = rcc.CartPoleDMEnvPool
-    report["adapter_mro"] = [c.__module__ + "." + c.__name__ for c in cls.__mro__]
     n = 3
     ids = np.arange(n, dtype=np.int32)
     done, trunc = np.array([0, 1, 1], bool), np.array([0, 0, 1], bool)
     obs = np.arange(4 * n, dtype=np.float32).reshape(n, 4)
     cols = [ids, ids, np.full(n, 7, np.int32), done, np.ones(n, np.float32),
             (~done).astype(np.float32), np.array([1, 2, 2], np.int32), trunc, obs]
-    ts = cls._to(None, cols, False, True)
+    ts = rcc.CartPoleDMEnvPool._to(None, cols, False, True)
     report["dm_fold"] = {
         "obs_is_same_object": ts.observation.obs is obs,
         "players_env_id": ts.observation.players.env_id.tolist(),
         "last": ts.last().tolist(), "reward": ts.reward.tolist(),
+        "step_type": [int(x) for x in ts.step_type],
     }
-    # constructing a pool goes through the reference's __init__ into OUR engine; without a
-    # GPU it must fail loudly from the engine (no CPU fallback), with one it must step
-    try:
-        env = envpool.make_gymnasium("CartPole-v1", num_envs=4, seed=3)
-        o, info = env.reset()
-        o2, rew, term, trunc_, info = env.step(np.array([0, 1, 0, 1], np.int32))
-        report["pool"] = {"ok": True, "obs_shape": list(o2.shape), "reward": rew.tolist(),
-                          "env_id": info["env_id"].tolist()}
-    except Exception as exc:  # noqa: BLE001
-        report["pool"] = {"ok": False, "error": f"{type(exc).__name__}: {exc}"}
-    print("REPORT " + json.dumps(report))
+    with open(GOLDEN, "w") as f:
+        json.dump(report, f, indent=1, sort_keys=True)
+        f.write("\n")
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -1,5 +1,8 @@
 """CPU: the oracle (oracle/ep_oracle.c) against the golden fixtures recorded from the
 reference itself, plus RNG known-answer tests.  This is what pins the oracle."""
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -58,21 +61,23 @@ def test_survey_known_answers():
 
 
 def test_oracle_matches_compiled_reference_when_present():
-    """When oracle/_ref (the reference compiled from /root/reference) is present, pin the
-    restatement against it directly on a fresh seed/action stream."""
-    from oracle import ref_lib
+    """The restatement against the reference's own AsyncEnvPool on a fresh seed/action
+    stream: every batch must match, bit for bit, the digest of the batch the reference
+    returned (golden/digests/ref_stream.npz, recorded by golden/make_golden.py)."""
     from oracle.oracle_lib import OraclePool
-    from helpers import REGISTERED, random_actions
+    from helpers import GOLDEN, REGISTERED, batch_digest, random_actions
 
-    if not ref_lib.available():
-        pytest.skip("oracle/_ref not built in this environment")
-    rng = np.random.default_rng(31)
+    rec = np.load(os.path.join(GOLDEN, "digests", "ref_stream.npz"))
+    meta = json.loads(str(rec["meta"]))
+    N, T = meta["num_envs"], meta["steps"]
+    rng = np.random.default_rng(meta["action_seed"])
     for task, (ms, iopt) in REGISTERED.items():
-        N, T = 32, 300
-        r = ref_lib.RefPool(task, N, seed=19, max_episode_steps=ms, iopt=iopt)
-        o = OraclePool(task, N, seed=19, max_episode_steps=ms, iopt=iopt)
-        assert_batch_equal(o.reset(), r.reset(), task, 0.0, f"{task} reset")
-        for t in range(T):
-            a = random_actions(task, rng, (N,))
-            assert_batch_equal(o.step(a), r.step(a), task, 0.0, f"{task} t={t}")
-        r.close()
+        acts = np.stack([random_actions(task, rng, (N,)) for _ in range(T)])
+        assert batch_digest({"actions": acts}) == int(rec[task + ":actions"][0]), \
+            f"{task}: the action stream is not the recorded one"
+        keys = meta["keys"][task]
+        o = OraclePool(task, N, seed=meta["seed"], max_episode_steps=ms, iopt=iopt)
+        got = [o.reset()] + [o.step(a) for a in acts]
+        got = [batch_digest({k: b[k] for k in keys}) for b in got]
+        bad = np.flatnonzero(np.array(got, dtype=np.uint64) != rec[task])
+        assert bad.size == 0, f"{task}: first differing batch {bad[0]} (0 = reset)"
